@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- CTC-CRF loss+grad frames/sec on synthetic (N,T,V) log-probs (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path (numerator + denominator forward-backward, loss and (N,T,V) gradient)
@@ -11,6 +11,8 @@ N=64 utterances per GPU, T=1500, V=218, fp32, T-compose-LM den graph H=20000/d=2
 scaling, no data-path collective) plus the path's single all-reduce of [sum cost, count].
 
 One JSON line on stdout (rank 0).  See DESIGN.md "Measurement" for how each field is obtained.
+--dump-outputs DIR writes what the timed path returned in its last timed step (see dump_outputs) so that two builds can
+be compared output for output: the inputs are seeded, identical from run to run for the same arguments.
 """
 from __future__ import annotations
 
@@ -54,7 +56,11 @@ def parse():
     ap.add_argument("--cpu-sample", default="auto", help="N,T of the CPU sample (default sized for ~15 s)")
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling block (global batches sharded over the ranks)")
     ap.add_argument("--strong-configs", default="5,4", help="which SURVEY configs the strong block runs (5: N=256 var-len; 4: N=128, 5M-arc graph)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's loss and gradient to DIR/<name>.npy (rank 0)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def peaks():
@@ -65,14 +71,41 @@ def peaks():
     return 6650.0, "fallback (B200_PROFILING.md)"
 
 
+_graph_dir = None
+
+
 def den_graph_file(H, d, V):
+    """The seeded synthetic den graph, written to a temporary directory of this process (removed at exit): the
+    tree may be read-only, and a fixed name in a shared /tmp could be another user's or another version's file."""
+    global _graph_dir
     from cat_b200 import fst
-    path = os.path.join(tempfile.gettempdir(), f"ccb_den_H{H}_d{d}_V{V}_r{os.environ.get('RANK', '0')}.fst")
+    if _graph_dir is None:
+        _graph_dir = tempfile.TemporaryDirectory(prefix="ccb_bench_")
+    path = os.path.join(_graph_dir.name, f"den_H{H}_d{d}_V{V}.fst")
     g = fst.make_synthetic_den(H, d, V, seed=7)
     if not os.path.exists(path):
-        fst.write_fst(path + ".tmp", g)
-        os.replace(path + ".tmp", path)
+        fst.write_fst(path, g)
     return path, g
+
+
+DUMP_BYTES = 48_000_000     # what dump_outputs writes at most, headers aside
+
+
+def dump_outputs(outdir, loss, grad):
+    """What a caller of the timed path receives, as float32 or float64 .npy files: loss.npy, and the (N,T,V) gradient,
+    as grad.npy when it fits DUMP_BYTES, otherwise as grad_rows.npy, the rows (n, t) of a fixed seeded sample, with
+    grad_row_index.npy holding their indices n*T + t (the headline gradient is 84 MB)."""
+    os.makedirs(outdir, exist_ok=True)
+    grad = torch.as_tensor(grad)
+    np.save(os.path.join(outdir, "loss.npy"), np.atleast_1d(torch.as_tensor(loss).detach().cpu().numpy()))
+    if grad.numel() * grad.element_size() <= DUMP_BYTES:
+        np.save(os.path.join(outdir, "grad.npy"), grad.detach().cpu().numpy())
+        return
+    rows = grad.detach().reshape(-1, grad.shape[-1])
+    n_keep = DUMP_BYTES // (8 + rows.shape[1] * rows.element_size())
+    idx = np.sort(np.random.default_rng(0).choice(rows.shape[0], n_keep, replace=False))
+    np.save(os.path.join(outdir, "grad_rows.npy"), rows[torch.from_numpy(idx).to(rows.device)].cpu().numpy())
+    np.save(os.path.join(outdir, "grad_row_index.npy"), idx.astype(np.float64))
 
 
 def synth_labels(N, T, V, seed, varlen=False):
@@ -156,13 +189,13 @@ CPU_SAMPLE_T = 32     # frames per utterance of the CPU legs' sample (the same i
 
 def cpu_port(graph, N, T, V, lamb, threads, seed=1234):
     """Times the fp64 oracle (oracle/ -- the CPU restatement; the reference has no CPU path) on a bounded
-    sample of the workload.  Returns (frames/s, seconds)."""
+    sample of the workload.  Returns (frames/s, seconds, loss, grad)."""
     from oracle import oracle
     y, labels, lens, ly = oracle.synth_batch(N, T, V, seed=seed)
     t0 = time.perf_counter()
-    oracle.ctc_crf(graph, y, labels, lens, ly, lamb, True, nthreads=threads)
+    loss, grad, _ = oracle.ctc_crf(graph, y, labels, lens, ly, lamb, True, nthreads=threads)
     dt = time.perf_counter() - t0
-    return float(lens.sum()) / dt, dt
+    return float(lens.sum()) / dt, dt, loss, grad
 
 
 def run_reference(args, rank):
@@ -183,9 +216,11 @@ def run_reference(args, rank):
     t0 = time.perf_counter()
     frames = 0
     for k in range(args.steps):
-        cpu_port(g, sN, sT, args.V, args.lamb, cores, seed=1234 + k)
+        _, _, loss, grad = cpu_port(g, sN, sT, args.V, args.lamb, cores, seed=1234 + k)
         frames += sN * sT
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, np.float64(loss), grad)
     v = frames / dt
     sample = f"N={sN},T={sT} slice of the workload per step (same den graph, V, lamb)"
     print(json.dumps({
@@ -235,12 +270,15 @@ def main():
     crit = ctc_crf.CTC_CRF_LOSS(lamb=args.lamb, size_average=True)
 
     host_s = [0.0, 0]   # host-side enqueue time of the resident steps (diagnostic: the GPU must never wait for it)
+    last = {}           # the outputs of the latest resident step (--dump-outputs)
 
     def step_resident():
         t0 = time.perf_counter()
         loss, grad, _ = _C.ctc_crf_loss_fwd(y, labels, lx, ly, args.lamb, True)
         host_s[0] += time.perf_counter() - t0
         host_s[1] += 1
+        if args.dump_outputs:
+            last["loss"], last["grad"] = loss, grad
         if world > 1:
             v = torch.stack([loss.reshape(()) * N, torch.tensor(float(N), device=dev)])
             dist.all_reduce(v)
@@ -272,10 +310,15 @@ def main():
     sampler = ClockSampler(local_rank)
     if rank == 0 and not os.environ.get("CCB_BENCH_NO_SAMPLER"):
         sampler.start()
-    ms_total = timed(step_resident, args.steps, max(args.warmup, 3))
+    try:
+        ms_total = timed(step_resident, args.steps, max(args.warmup, 3))
+    finally:            # never leave nvidia-smi running behind
+        clocks = sampler.stop() if rank == 0 else None
     launches = _C.launch_count() - timed.launches_before
-    clocks = sampler.stop() if rank == 0 else None
     ms_per_step = ms_total / args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last["loss"], last["grad"])
+    last.clear()
     value = world * frames_per_step / (ms_per_step * 1e-3)
 
     # ---- e2e: public API, host buffers, H2D of the step's logits + D2H of the loss inside the timed region ----
@@ -474,7 +517,7 @@ def main():
                 else:
                     sN, sT = [int(x) for x in args.cpu_sample.split(",")]
                 cores = min(cores, sN)    # the port parallelises over utterances: threads actually used
-                v, dt = cpu_port(graph, sN, sT, V, args.lamb, cores)
+                v, dt, _, _ = cpu_port(graph, sN, sT, V, args.lamb, cores)
                 cpu_baseline = {"value": v, "unit": UNIT, "cores": cores, "cpu_model": cpu_model(), "kind": "port", "seconds": dt,
                                 "sample": f"fp64 oracle port (reference has no CPU path), N={sN},T={sT} slice, same den graph/V/lamb, {cores} threads"}
         out = {
